@@ -38,6 +38,8 @@ RAYS, SPR = 4096, 512
 SEGMENTS = tuple(int(x) for x in os.environ.get("HRF_BENCH_SEGMENTS", "50").split(","))
 ALG_BYTES_FWD = 3084          # SURVEY 8d: 2048 B table gathers + 1024 B vector taps + 12 B stream, per sample
 ALG_BYTES_SCATTER = 6144      # SURVEY 8d backward convention: table-gradient RMW 2 x 2048 B + vector-gradient RMW 2 x 1024 B
+DUMP_SAMPLE = 1 << 20        # --dump-outputs: larger outputs are written as a fixed seeded sample of this many elements
+DUMP_LIMIT = 64 << 20        # bytes, all files together
 METRIC = {"render": "render_rays_per_s", "train": "train_rays_per_s", "image": "render_mpix_per_s", "sweep": "render_mpix_per_s"}
 UNIT = {"render": "rays/s", "train": "rays/s", "image": "Mpix/s", "sweep": "Mpix/s"}
 
@@ -127,6 +129,28 @@ class ClockSampler:
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_outputs(directory, arrays):
+    """Writes each output array as DIR/<name>.npy in float32 (float64 stays float64).  An array of more than DUMP_SAMPLE
+    elements is flattened and reduced to the elements at DUMP_SAMPLE flat indices drawn once from a generator seeded with
+    0 (sorted), the same in every run, so two builds can be compared element by element."""
+    import numpy as np
+
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    total = 0
+    for name, x in arrays.items():
+        x = x.detach()
+        if x.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(x.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort()[0]
+            x = x.reshape(-1)[idx.to(x.device)]
+        a = x.cpu().numpy()
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        total += a.nbytes
+        if total > DUMP_LIMIT:
+            raise SystemExit(f"--dump-outputs: more than {DUMP_LIMIT >> 20} MB of outputs")
+        np.save(out / f"{name}.npy", a)
 
 
 def build_workload(device, seed):
@@ -227,6 +251,8 @@ def run_image(args, dev, rank, world):
     if world > 1:
         dist.all_reduce(dt, op=dist.ReduceOp.MAX)
     clk = clocks.stop()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"image_tile": img})
     if rank == 0:
         mpix = W * H * args.steps / float(dt.item()) / 1e6
         frac = float((host[: e - s].abs().sum(1) > 0).float().mean())
@@ -286,6 +312,8 @@ def run_sweep(args, dev, rank, world, model, frames, renderer, clocks, W, H, G):
     if world > 1:
         dist.all_reduce(dt, op=dist.ReduceOp.MAX)
     clk = clocks.stop()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"image": img})
     if rank == 0:
         images = args.steps * world
         mpix = W * H * images / float(dt.item()) / 1e6
@@ -311,6 +339,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-companions", action="store_true",
                     help="do not append the render / full-image numbers to the default train line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -356,13 +386,15 @@ def main():
         trainer.profile = True
     g = {k: v.to(dev).contiguous() for k, v in b.items() if k in ("o", "d", "frames", "t", "ri", "rgba")}
     n = g["t"].shape[0]
-    bg = torch.rand(RAYS, 3, device=dev)
+    bg = torch.rand(RAYS, 3, device=dev, generator=torch.Generator(device=dev).manual_seed(7))
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)   # > 126 MB L2
     off_all = ray_offsets(g["ri"], RAYS)
     launches = {"n": 0}
+    rendered = {}
 
     def step_render(ev=None):
-        render_fused(model, g["o"], g["d"], g["frames"], g["t"], g["ri"], RAYS, bg, ray_offsets_dev=off_all)
+        rendered["color"], rendered["weights_sum"] = render_fused(model, g["o"], g["d"], g["frames"], g["t"], g["ri"], RAYS, bg,
+                                                                  ray_offsets_dev=off_all)
         if ev is not None:
             ev.record()
         launches["n"] += 2
@@ -419,6 +451,19 @@ def main():
         if world > 1:   # every rank draws its own ray batch: report the spread of the per-rank work
             dist.all_reduce(kept_ranks, op=dist.ReduceOp.MAX)
         kept_max, kept_min = float(kept_ranks[0].item()), -float(kept_ranks[1].item())
+    if args.dump_outputs:
+        if args.mode == "render":
+            outputs = dict(rendered)
+        else:
+            # what a caller of FusedTrainer.step gets from the last step: the loss, the surviving sample count and the
+            # parameters it updated in place (with the p2p exchange, each rank's fp32 tables are current only in its shard)
+            if world > 1:
+                trainer.gather_master_parameters()
+            names = {id(p): name for name, p in model.named_parameters()}
+            outputs = {"loss": trainer.last["loss"].reshape(1), "samples_after_prune": trainer.last["samples"].reshape(1).double()}
+            outputs.update({names[id(p)]: p for p in model.hot_parameters()})
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
 
     # ---- e2e through the public API with pinned host buffers -------------------------------------
     host = {k: b[k].contiguous().pin_memory() for k in ("o", "d", "frames", "t", "ri", "rgba")}
@@ -502,7 +547,7 @@ def main():
     e2e_loop(5)
     barrier()
     t0 = time.perf_counter()
-    k_e2e = max(50, args.steps)
+    k_e2e = args.steps
     e2e_loop(k_e2e)
     barrier()
     e2e_s = time.perf_counter() - t0
@@ -582,7 +627,7 @@ def main():
             # BASELINE.json's metric is a pair ("train rays/sec & render Mpix/s"): the other two workloads run right after
             # (each in its own process, own timed region, same rules) and are attached so one run reports all three.
             line["render"] = companion_line("render", args.steps)
-            line["image"] = companion_line("image", 5)
+            line["image"] = companion_line("image", args.steps)
             line["config"]["render_rays_per_s"] = line["render"].get("value")
             line["config"]["render_mpix_per_s"] = line["image"].get("value")
         print(json.dumps(line))

@@ -1,20 +1,21 @@
-"""Generates tests/golden/reference_host.npz by IMPORTING the reference (read-only at
-/root/reference) and running its pure-torch first-party functions on seeded inputs:
+"""Generates tests/golden/reference_host.npz by IMPORTING the reference (the checkout HUMANRF_REFERENCE
+names, read-only) and running its pure-torch first-party functions on seeded inputs:
 
   humanrf/input.py:10-55                 merge_input_batches (incl. the sample-budget cut-off)
   humanrf/utils/activation.py:6-39       truncated_exp forward / backward
   humanrf/utils/loss.py:4-10             bce_loss
   actorshq/dataset/camera_data.py:93-102 projection_matrix_world2pixel -> inverse_krs (data_loader.py:194-207)
 
-Run here (the reference does not exist on the GPU box):  python tests/golden/make_golden.py
+Run:  HUMANRF_REFERENCE=/path/to/humanrf python tests/golden/make_golden.py
 """
+import os
 import sys
 from pathlib import Path
 
 import numpy as np
 import torch
 
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.environ["HUMANRF_REFERENCE"])
 from actorshq.dataset.camera_data import CameraData  # noqa: E402
 from actorshq.dataset.input_batch import InputBatch  # noqa: E402
 from humanrf.input import merge_input_batches  # noqa: E402

@@ -1,13 +1,16 @@
 """Generates tests/golden/partitioning.npz by running the REFERENCE's compute_adaptive_segment_sizes
-(/root/reference/humanrf/adaptive_temporal_partitioning.py) on synthetic occupancy sequences.  Runs only in the build
-container (needs /root/reference); the fixture and this script are committed."""
+(humanrf/adaptive_temporal_partitioning.py of the reference checkout HUMANRF_REFERENCE names) on synthetic occupancy
+sequences.  Run:  HUMANRF_REFERENCE=/path/to/humanrf python tests/golden/make_partitioning_golden.py"""
+import os
 import sys
 import types
+from pathlib import Path
 
 import numpy as np
 
-sys.path.insert(0, "/root/reference")
-sys.path.insert(0, "/root/repo")
+HERE = Path(__file__).resolve().parent
+sys.path.insert(0, os.environ["HUMANRF_REFERENCE"])
+sys.path.insert(0, str(HERE.parent.parent))
 # the reference module imports VolumetricDataset only for a type annotation; avoid its heavy imports
 stub = types.ModuleType("actorshq.dataset.volumetric_dataset")
 stub.VolumetricDataset = object
@@ -16,7 +19,7 @@ for name in ("actorshq", "actorshq.dataset"):
 sys.modules["actorshq.dataset.volumetric_dataset"] = stub
 from humanrf.adaptive_temporal_partitioning import compute_adaptive_segment_sizes  # noqa: E402
 
-sys.path.insert(0, "/root/repo/tests")
+sys.path.insert(0, str(HERE.parent))
 from scene import occupancy_sequence  # noqa: E402
 
 
@@ -37,4 +40,4 @@ for name, n, speed, thr in cases:
     out[name + "_sizes"] = np.asarray(sizes, np.int32)
     out[name + "_args"] = np.asarray([n, -1.0 if speed is None else speed, thr, len(name) * 7 + n], np.float64)
     print(name, sizes)
-np.savez_compressed("/root/repo/tests/golden/partitioning.npz", **out)
+np.savez_compressed(HERE / "partitioning.npz", **out)

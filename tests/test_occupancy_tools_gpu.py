@@ -1,9 +1,6 @@
 """SURVEY 8f-4 on the GPU: visual-hull carving bit-exact against the oracle and statistically against the reference's
-own extension (oracle/_ref); adaptive temporal partitioning against the reference's golden decisions."""
-import importlib
-import sys
-from pathlib import Path
-
+own extension (its answer stored in tests/golden/reference_cuda.npz); adaptive temporal partitioning against the
+reference's golden decisions."""
 import numpy as np
 import pytest
 import torch
@@ -11,9 +8,9 @@ import torch
 from oracle import occupancy_tools as O
 from scene import carve_scene, occupancy_sequence
 from test_occupancy_tools_cpu import golden_cases
+from test_ref_parity_gpu import reference_outputs
 
 pytestmark = pytest.mark.gpu
-REF = Path(__file__).resolve().parent.parent / "oracle" / "_ref"
 
 
 def _carve(sc, thr, G, cuda):
@@ -39,24 +36,26 @@ def test_carve_rejects_wrong_mask_size(cuda):
         _carve(dict(sc, width=31), 1, 8, cuda)
 
 
-def test_carve_vs_reference_extension(cuda):
-    """Full-size carve (G=256, 24 cameras) against the reference's kernel built from its unmodified source.  The
-    reference is compiled with --use_fast_math (approximate divides), so a voxel whose projection lands within an ulp
-    of a pixel boundary may sample a neighbouring mask pixel: a handful of voxels out of 16.7 M."""
-    if not (REF / "occupancy_grid_generation_native.so").exists():
-        pytest.skip("oracle/_ref/occupancy_grid_generation_native.so not built")
-    if str(REF) not in sys.path:
-        sys.path.insert(0, str(REF))
-    ref = importlib.import_module("occupancy_grid_generation_native")
+def reference_carve_args(device):
+    """Full-size carve: G=256, 24 cameras of 512x384, threshold 20."""
     sc = carve_scene(num_cameras=24, width=512, height=384, seed=5)
-    G, thr = 256, 20
-    args = (torch.from_numpy(sc["masks"]).to(cuda), torch.from_numpy(sc["projection_matrices"]).to(cuda),
-            torch.from_numpy(sc["landscape"]).to(cuda), thr, G, 512, 384)
-    want = ref.generate_from_masks(*args)
+    return (torch.from_numpy(sc["masks"]).to(device), torch.from_numpy(sc["projection_matrices"]).to(device),
+            torch.from_numpy(sc["landscape"]).to(device), 20, 256, 512, 384)
+
+
+def test_carve_vs_reference_extension(cuda):
+    """Full-size carve (G=256, 24 cameras) against the reference's kernel built from its unmodified source (it returns
+    0 or 255 per voxel; the occupied voxels are stored as a bit mask).  The reference is compiled with --use_fast_math
+    (approximate divides), so a voxel whose projection lands within an ulp of a pixel boundary may sample a
+    neighbouring mask pixel: a handful of voxels out of 16.7 M."""
+    args = reference_carve_args(cuda)
+    G = args[4]
+    want = torch.from_numpy(np.unpackbits(reference_outputs()["carve_occupied_bits"])[:G ** 3].reshape(G, G, G) * 255).to(cuda)
     from humanrf_b200.toolbox import occupancy_grid_generation_native as ours
 
     got = ours.generate_from_masks(*args)
     torch.cuda.synchronize()
+    assert got.shape == want.shape and got.dtype == want.dtype
     diff = int((want != got).sum())
     occ = int((want == 255).sum())
     def ms(fn):
@@ -67,8 +66,7 @@ def test_carve_vs_reference_extension(cuda):
         e1.record(); torch.cuda.synchronize()
         return e0.elapsed_time(e1) / 5
 
-    print(f"carve vs reference: {diff} of {G ** 3} voxels differ, {occ} occupied; "
-          f"ours {ms(lambda: ours.generate_from_masks(*args)):.3f} ms, reference {ms(lambda: ref.generate_from_masks(*args)):.3f} ms")
+    print(f"carve vs reference: {diff} of {G ** 3} voxels differ, {occ} occupied; ours {ms(lambda: ours.generate_from_masks(*args)):.3f} ms")
     assert 0 < occ < G ** 3 and diff <= 2e-5 * G ** 3
 
 

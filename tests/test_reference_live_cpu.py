@@ -1,9 +1,11 @@
-"""Differential tests against the LIVE reference (imported read-only from /root/reference) on randomized inputs, for the
-first-party pure-Python pieces of the path.  They complement the frozen goldens of tests/golden/ (which also run on the
-GPU box, where the reference does not exist): here every run draws many more cases.  Skipped when the reference is
-not mounted."""
+"""Differential tests against the reference's first-party pure-Python pieces of the path, on randomized inputs.  The
+reference's answers for exactly these inputs are stored in tests/golden/reference_python.json and .npz (written by
+tests/golden/make_reference_python_golden.py from a reference checkout), so the comparisons run without one: the
+inputs are rebuilt here from the same seeds and our side is run live."""
 import dataclasses
-import sys
+import functools
+import hashlib
+import json
 import types
 from pathlib import Path
 
@@ -11,40 +13,23 @@ import numpy as np
 import pytest
 import torch
 
-REF = Path("/root/reference")
-pytestmark = pytest.mark.skipif(not REF.exists(), reason="reference checkout not present (GPU box)")
+GOLDEN = Path(__file__).resolve().parent / "golden"
+
+
+@functools.lru_cache(maxsize=None)
+def _golden():
+    return json.loads((GOLDEN / "reference_python.json").read_text()), dict(np.load(GOLDEN / "reference_python.npz"))
 
 
 @pytest.fixture(scope="module")
 def ref():
-    """The reference's importable modules.  Imported under their own names, so anything of ours that was shadowed is
-    restored afterwards."""
-    saved = {k: v for k, v in sys.modules.items() if k.split(".")[0] in ("humanrf", "actorshq")}
-    for k in saved:
-        del sys.modules[k]
-    sys.path.insert(0, str(REF))
-    try:
-        import actorshq.dataset.input_batch as ib
-        import humanrf.input as inp
-        import humanrf.scene_representation.query_io as qio
-        import humanrf.utils.activation as act
-        import humanrf.utils.loss as loss
-        # adaptive_temporal_partitioning imports VolumetricDataset only for an annotation (needs cv2 etc.): stub it
-        if "actorshq.dataset.volumetric_dataset" not in sys.modules:
-            stub = types.ModuleType("actorshq.dataset.volumetric_dataset")
-            stub.VolumetricDataset = object
-            sys.modules["actorshq.dataset.volumetric_dataset"] = stub
-        import humanrf.adaptive_temporal_partitioning as atp
-        yield types.SimpleNamespace(ib=ib, inp=inp, qio=qio, act=act, loss=loss, atp=atp)
-    finally:
-        sys.path.remove(str(REF))
-        for k in [k for k in sys.modules if k.split(".")[0] in ("humanrf", "actorshq")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
+    """The reference's stored answers: (JSON document, arrays)."""
+    return _golden()
 
 
-def _surface(cls):
-    fields = [(f.name, f.default) for f in dataclasses.fields(cls)]
+def surface(cls):
+    """Dataclass fields with their defaults, and public members (JSON-able: an absent default is "MISSING")."""
+    fields = [[f.name, "MISSING" if f.default is dataclasses.MISSING else repr(f.default)] for f in dataclasses.fields(cls)]
     return fields, sorted(m for m in dir(cls) if not m.startswith("_"))
 
 
@@ -52,9 +37,9 @@ def test_dataclass_surfaces_match(ref):
     from humanrf_b200.dataset.input_batch import InputBatch
     from humanrf_b200.scene_representation.query_io import QueryInput, QueryOutput
 
-    assert _surface(InputBatch) == _surface(ref.ib.InputBatch)
-    assert _surface(QueryInput) == _surface(ref.qio.QueryInput)
-    assert _surface(QueryOutput) == _surface(ref.qio.QueryOutput)
+    want = ref[0]["surfaces"]
+    for cls in (InputBatch, QueryInput, QueryOutput):
+        assert list(surface(cls)) == want[cls.__name__], cls.__name__
 
 
 FIELDS = ["ray_origins", "ray_directions", "minmaxes", "rgba", "ray_masks", "frame_numbers", "unique_frame_numbers",
@@ -77,75 +62,75 @@ def _batch(cls, rng, num_rays, masked):
                width=64, height=48)
 
 
+def merge_cases(cls):
+    """60 random configurations of merge_input_batches, batches built with `cls`: (case, batches, budget, total samples)."""
+    rng = np.random.default_rng(7)
+    for case in range(60):
+        nb = int(rng.integers(1, 5))
+        specs = [(int(rng.integers(1, 30)), int(rng.integers(0, 5))) for _ in range(nb)]
+        r2 = np.random.default_rng(int(rng.integers(0, 2 ** 31)))
+        batches = [_batch(cls, r2, *s) for s in specs]
+        total = sum(b.sample_distances.shape[0] for b in batches)
+        yield case, batches, [None, max(1, total // 2), max(1, total - 1), total, total + 5, 1][case % 6], total
+
+
+def merged_fields(out):
+    """Each field of a merged batch as "dtype shape digest", the digest a 96-bit prefix of the SHA-256 of its bytes
+    (unique frame numbers sorted first)."""
+    res = {}
+    for f in FIELDS:
+        x = getattr(out, f)
+        if f == "unique_frame_numbers":
+            x = torch.sort(x.reshape(-1))[0]
+        digest = hashlib.sha256(np.ascontiguousarray(x.numpy()).tobytes()).hexdigest()[:24]
+        res[f] = f"{str(x.dtype).replace('torch.', '')} {'x'.join(map(str, x.shape))} {digest}"
+    return res
+
+
 def test_merge_input_batches_randomized(ref):
     """input.py:10-55 incl. the sample-budget cut-off and its `cumsum < cutoff` behaviour, 60 random configurations."""
     from humanrf_b200.dataset.input_batch import InputBatch
     from humanrf_b200.input import merge_input_batches
 
-    rng = np.random.default_rng(7)
+    want = ref[0]["merge"]
     checked_cut = 0
-    for case in range(60):
-        nb = int(rng.integers(1, 5))
-        specs = [(int(rng.integers(1, 30)), int(rng.integers(0, 5))) for _ in range(nb)]
-        seed = int(rng.integers(0, 2 ** 31))
-        total = None
-        outs = []
-        for cls, fn in ((ref.ib.InputBatch, ref.inp.merge_input_batches), (InputBatch, merge_input_batches)):
-            r2 = np.random.default_rng(seed)
-            batches = [_batch(cls, r2, *s) for s in specs]
-            total = sum(b.sample_distances.shape[0] for b in batches)
-            budget = [None, max(1, total // 2), max(1, total - 1), total, total + 5, 1][case % 6]
-            outs.append(fn(batches, budget))
-        a, b = outs
+    for case, batches, budget, total in merge_cases(InputBatch):
         if budget is not None and budget < total:
             checked_cut += 1
+        out = merge_input_batches(batches, budget)
+        got = merged_fields(out)
         for f in FIELDS:
-            x, y = getattr(a, f), getattr(b, f)
-            if f == "unique_frame_numbers":
-                x, y = torch.sort(x.reshape(-1))[0], torch.sort(y.reshape(-1))[0]
-            assert x.dtype == y.dtype and x.shape == y.shape and torch.equal(x, y), (case, f)
-        assert (a.width, a.height) == (b.width, b.height)
-    assert checked_cut >= 15
+            assert got[f] == want[case]["fields"][f], (case, f)
+        assert [out.width, out.height] == want[case]["size"]
+    assert len(want) == 60 and checked_cut >= 15
+
+
+def truncated_exp_inputs():
+    g = torch.Generator().manual_seed(3)
+    for scale in (1.0, 9.0, 30.0):
+        yield scale, torch.randn(513, generator=g) * scale, torch.randn(513, generator=g)
+    pred = torch.rand(777, 1, generator=g) * 1.6 - 0.3
+    yield "bce", pred, (torch.rand(777, 1, generator=g) > 0.4).float()
 
 
 def test_truncated_exp_and_bce_randomized(ref):
     from humanrf_b200.utils.activation import truncated_exp
     from humanrf_b200.utils.loss import bce_loss
 
-    g = torch.Generator().manual_seed(3)
-    for scale in (1.0, 9.0, 30.0):
-        x = torch.randn(513, generator=g) * scale
-        dy = torch.randn(513, generator=g)
-        outs = []
-        for fn in (ref.act.truncated_exp, truncated_exp):
-            xi = x.clone().requires_grad_(True)
-            y = fn(xi)
-            y.backward(dy)
-            outs.append((y.detach(), xi.grad))
-        assert torch.equal(outs[0][0], outs[1][0]) and torch.equal(outs[0][1], outs[1][1])
-    pred = torch.rand(777, 1, generator=g) * 1.6 - 0.3
-    target = (torch.rand(777, 1, generator=g) > 0.4).float()
-    assert torch.equal(ref.loss.bce_loss(pred, target), bce_loss(pred, target))
+    arrays = ref[1]
+    for scale, x, dy in truncated_exp_inputs():
+        if scale == "bce":
+            assert torch.equal(bce_loss(x, dy), torch.from_numpy(arrays["bce_out"]))
+            continue
+        xi = x.clone().requires_grad_(True)
+        y = truncated_exp(xi)
+        y.backward(dy)
+        assert torch.equal(y.detach(), torch.from_numpy(arrays[f"texp_{scale:g}_y"]))
+        assert torch.equal(xi.grad, torch.from_numpy(arrays[f"texp_{scale:g}_dx"]))
 
 
-def test_segment_size_rules_and_partitioning_randomized(ref):
-    """adaptive_temporal_partitioning.py:28-107 against the oracle restatement (the GPU implementation is compared with
-    the same reference decisions through tests/golden/partitioning.npz)."""
-    from humanrf_b200 import adaptive_temporal_partitioning as ours
-    from oracle import occupancy_tools as O
-
-    assert ours.PREDEFINED_SEGMENT_SIZES == ref.atp.PREDEFINED_SEGMENT_SIZES == O.PREDEFINED_SEGMENT_SIZES
-    for n in range(1, 260):
-        assert ours.get_segment_size(n) == ref.atp.get_segment_size(n) == O.get_segment_size(n)
-        assert ours.get_final_segment_size(n) == ref.atp.get_final_segment_size(n) == O.get_final_segment_size(n)
-
-    class DS:
-        def __init__(self, grids):
-            self.grids = grids
-
-        def get_occupancy_grid(self, frame_number):
-            return self.grids[frame_number].copy()       # the reference ORs into the first grid of a cluster in place
-
+def partitioning_cases():
+    """12 random occupancy sequences (occasional growth, jumps) and thresholds: (grids, threshold)."""
     rng = np.random.default_rng(11)
     for case in range(12):
         n = int(rng.integers(3, 140))
@@ -157,85 +142,56 @@ def test_segment_size_rules_and_partitioning_randomized(ref):
             if rng.random() < 0.03:
                 cur = rng.random(cur.shape) < 0.2             # a jump
             grids.append((cur * 255).astype(np.uint8))
-        thr = [1.05, 1.25, 2.0][case % 3]
-        import contextlib
-        import io
-
-        with contextlib.redirect_stderr(io.StringIO()):      # tqdm bar
-            want = ref.atp.compute_adaptive_segment_sizes(DS(grids), list(range(n)), thr)
-        assert O.compute_adaptive_segment_sizes(grids, thr) == want, case
+        yield grids, [1.05, 1.25, 2.0][case % 3]
 
 
-_MODEL_CACHE = {}
+def test_segment_size_rules_and_partitioning_randomized(ref):
+    """adaptive_temporal_partitioning.py:28-107 against the oracle restatement (the GPU implementation is compared with
+    the same reference decisions through tests/golden/partitioning.npz)."""
+    from humanrf_b200 import adaptive_temporal_partitioning as ours
+    from oracle import occupancy_tools as O
+
+    want = ref[0]["partitioning"]
+    assert list(ours.PREDEFINED_SEGMENT_SIZES) == want["predefined"] == list(O.PREDEFINED_SEGMENT_SIZES)
+    for n in range(1, 260):
+        assert ours.get_segment_size(n) == want["segment_size"][n - 1] == O.get_segment_size(n)
+        assert ours.get_final_segment_size(n) == want["final_segment_size"][n - 1] == O.get_final_segment_size(n)
+    cases = list(partitioning_cases())
+    assert len(cases) == len(want["sizes"])
+    for case, (grids, thr) in enumerate(cases):
+        assert O.compute_adaptive_segment_sizes(grids, thr) == want["sizes"][case], case
 
 
-def _import_reference_model():
-    """The reference's HumanRF with `tinycudann` and its compiled extension stubbed out: the stubs only RECORD the
-    configs they are constructed with and own one flat `.params` (sized by our layout rule -- sizes of tcnn tensors are
-    therefore not evidence, the configs / names / first-party tensors are)."""
-    from humanrf_b200.scene_representation.grid_layout import GridLayout, MLP_SIGMA_PARAMS, mlp_color_params
-
-    if _MODEL_CACHE:                       # the module stays bound to the stub classes (and their log) of its first import
-        _MODEL_CACHE["calls"].clear()
-        sys.modules["tinycudann"] = _MODEL_CACHE["tcnn"]
-        sys.modules["humanrf.scene_representation.humanrf"] = _MODEL_CACHE["module"]
-        return _MODEL_CACHE["module"], _MODEL_CACHE["calls"]
-    calls = []
-
-    class _Flat(torch.nn.Module):
-        def __init__(self, n):
-            super().__init__()
-            self.params = torch.nn.Parameter(torch.zeros(n))
-
-    class Encoding(_Flat):
-        def __init__(self, n_input_dims, encoding_config, **kw):
-            calls.append(("Encoding", n_input_dims, dict(encoding_config)))
-            c = encoding_config
-            fin = c["base_resolution"] * c["per_level_scale"] ** (c["n_levels"] - 1)
-            super().__init__(GridLayout(c["log2_hashmap_size"], c["n_levels"], c["base_resolution"], int(round(fin))).n_params)
-
-    class Network(_Flat):
-        def __init__(self, n_input_dims, n_output_dims, network_config, **kw):
-            calls.append(("Network", n_input_dims, n_output_dims, dict(network_config)))
-            super().__init__(MLP_SIGMA_PARAMS)
-
-    class NetworkWithInputEncoding(_Flat):
-        def __init__(self, n_input_dims, n_output_dims, encoding_config, network_config, **kw):
-            calls.append(("NetworkWithInputEncoding", n_input_dims, n_output_dims, dict(encoding_config), dict(network_config)))
-            super().__init__(mlp_color_params(n_input_dims - 18))
-
-    tcnn = types.ModuleType("tinycudann")
-    tcnn.Encoding, tcnn.Network, tcnn.NetworkWithInputEncoding = Encoding, Network, NetworkWithInputEncoding
-    sys.modules["tinycudann"] = tcnn
-    sys.modules["humanrf.scene_representation.tensor_composition_native"] = types.ModuleType("tensor_composition_native")
-    import humanrf.scene_representation.humanrf as ref_model
-
-    _MODEL_CACHE.update(module=ref_model, calls=calls, tcnn=tcnn)
-    return ref_model, calls
+MODEL_CASES = [((50,), 15, 50, 0), ((25, 12, 100, 6), 0, 140, 2), ((6, 6), 3, 9, 0)]
 
 
-@pytest.mark.parametrize("segment_sizes,first,count,cam_emb", [((50,), 15, 50, 0), ((25, 12, 100, 6), 0, 140, 2), ((6, 6), 3, 9, 0)])
-def test_model_constructor_against_the_reference(ref, segment_sizes, first, count, cam_emb):
-    """humanrf.py:68-156 + decomposition4d.py:73-122 run for real (only tcnn is a recording stub): frame LUTs, per-segment
-    hash-map sizes, encoding / network configs, state-dict key names and the shapes of the first-party tensors."""
-    from humanrf_b200.scene_representation.grid_layout import GridLayout
-    from humanrf_b200.scene_representation.humanrf import HumanRF
+def model_case_key(segment_sizes, first, count, cam_emb):
+    return f"{'-'.join(map(str, segment_sizes))}_{first}_{count}_{cam_emb}"
+
+
+def model_kwargs(cam_emb):
     from humanrf_b200.synthetic import MODEL_KW
 
-    try:
-        ref_model, calls = _import_reference_model()
-        frames = tuple(range(first, first + count))
-        kw = {**MODEL_KW, "camera_embedding_dim": cam_emb, "temporal_partitioning": "adaptive", "fixed_segment_size": 6}
-        theirs = ref_model.HumanRF(sorted_frame_numbers=frames, segment_sizes=segment_sizes, **kw)
-        ours = HumanRF(sorted_frame_numbers=frames, segment_sizes=segment_sizes, **kw)
-    finally:
-        sys.modules.pop("tinycudann", None)
+    return {**MODEL_KW, "camera_embedding_dim": cam_emb, "temporal_partitioning": "adaptive", "fixed_segment_size": 6}
+
+
+@pytest.mark.parametrize("segment_sizes,first,count,cam_emb", MODEL_CASES)
+def test_model_constructor_against_the_reference(ref, segment_sizes, first, count, cam_emb):
+    """humanrf.py:68-156 + decomposition4d.py:73-122 as the reference ran them (only tcnn was a recording stub): frame LUTs,
+    per-segment hash-map sizes, encoding / network configs, state-dict key names and the shapes of the first-party
+    tensors."""
+    from humanrf_b200.scene_representation.grid_layout import GridLayout
+    from humanrf_b200.scene_representation.humanrf import HumanRF
+
+    key = model_case_key(segment_sizes, first, count, cam_emb)
+    theirs, arrays = ref[0]["model"][key], ref[1]
+    ours = HumanRF(sorted_frame_numbers=tuple(range(first, first + count)), segment_sizes=segment_sizes, **model_kwargs(cam_emb))
     # frame -> segment / local-time look-up tables
-    assert torch.equal(ours.frame_numbers_to_segment_numbers, theirs.frame_numbers_to_segment_numbers)
-    assert torch.equal(ours.frame_numbers_to_normalized_local_frame_numbers, theirs.frame_numbers_to_normalized_local_frame_numbers)
-    assert (ours.num_frames, ours.num_segments, ours.total_feature_dim, ours.density_scale) == \
-           (theirs.num_frames, theirs.num_segments, theirs.total_feature_dim, theirs.density_scale)
+    for name in ("frame_numbers_to_segment_numbers", "frame_numbers_to_normalized_local_frame_numbers"):
+        assert torch.equal(getattr(ours, name), torch.from_numpy(arrays[f"model_{key}_{name}"])), name
+    assert [ours.num_frames, ours.num_segments, ours.total_feature_dim, ours.density_scale] == theirs["scalars"]
     # what the reference asks tcnn for, segment by segment
+    calls = theirs["calls"]
     enc = [c for c in calls if c[0] == "Encoding"]
     assert len(enc) == 4 * len(segment_sizes)
     for s, fg in enumerate(ours.feature_grids):
@@ -246,48 +202,19 @@ def test_model_constructor_against_the_reference(ref, segment_sizes, first, coun
             assert cfg["base_resolution"] == 32 and np.float32(cfg["per_level_scale"]) == np.float32(np.exp(np.log(2048 / 32) / 15))
             assert GridLayout(cfg["log2_hashmap_size"]).n_params == fg.layout.n_params
     net = [c for c in calls if c[0] == "Network"][0]
-    assert net[1:3] == (32, 16) and net[3] == {"otype": "FullyFusedMLP", "activation": "ReLU", "output_activation": "None",
+    assert net[1:3] == [32, 16] and net[3] == {"otype": "FullyFusedMLP", "activation": "ReLU", "output_activation": "None",
                                               "n_neurons": 64, "n_hidden_layers": 1}
     col = [c for c in calls if c[0] == "NetworkWithInputEncoding"][0]
-    assert col[1:3] == (18 + cam_emb, 3) and col[4]["output_activation"] == "Sigmoid" and col[4]["n_hidden_layers"] == 2
+    assert col[1:3] == [18 + cam_emb, 3] and col[4]["output_activation"] == "Sigmoid" and col[4]["n_hidden_layers"] == 2
     assert col[3]["nested"][0] == {"n_dims_to_encode": 3, "otype": "SphericalHarmonics", "degree": 4}
     # state dict: same keys in the same order, same shapes (first-party tensors: vectors, LUT buffers, embeddings)
-    a, b = ours.state_dict(), theirs.state_dict()
-    assert list(a.keys()) == list(b.keys())
-    for k in a:
-        assert a[k].shape == b[k].shape and a[k].dtype == b[k].dtype, k
+    assert [[k, list(v.shape), str(v.dtype)] for k, v in ours.state_dict().items()] == theirs["state_dict"]
     # optimiser parameter groups (humanrf.py:210-220)
-    ga, gb = ours.get_params(1e-2), theirs.get_params(1e-2)
-    assert [len(list(g["params"])) for g in ga] == [len(list(g["params"])) for g in gb] and [g["lr"] for g in ga] == [g["lr"] for g in gb]
+    assert [[len(list(g["params"])), g["lr"]] for g in ours.get_params(1e-2)] == theirs["param_groups"]
 
 
-def test_prune_and_render_glue_against_the_reference(ref):
-    """The reference's own prune_samples / render / merge_render_outputs (volume_rendering.py:26-150) executed on the CPU
-    with `nerfacc` replaced by the oracle's restatement of its three functions and a closed-form stand-in for the scene
-    representation: pins everything the oracle restates AROUND nerfacc (positions, jitter, alpha, t_ends = t + step,
-    mask application, background blend, output shapes).  nerfacc's own arithmetic stays unpinned."""
-    from helpers import synthetic_rays
-    from humanrf_b200.volume_rendering import RenderOutput as OurRenderOutput
-    from oracle import rendering as R
-
-    nerfacc = types.ModuleType("nerfacc")
-    nerfacc.render_visibility = lambda alphas, ray_indices, early_stop_eps, alpha_thre, n_rays: \
-        R.render_visibility(alphas, ray_indices, early_stop_eps, alpha_thre)
-
-    def render_weight_from_density(t_starts, t_ends, sigmas, ray_indices, n_rays):
-        sdt = sigmas.reshape(-1) * (t_ends - t_starts).reshape(-1)
-        return (torch.exp(-R._exclusive_by_ray(sdt, ray_indices, "sum")) * (1.0 - torch.exp(-sdt))).unsqueeze(-1)
-
-    nerfacc.render_weight_from_density = render_weight_from_density
-    nerfacc.accumulate_along_rays = lambda weights, ray_indices, values=None, n_rays=None: R.accumulate(weights, ray_indices, values, n_rays)
-    try:
-        _import_reference_model()
-        sys.modules["nerfacc"] = nerfacc
-        import humanrf.volume_rendering as vr
-    finally:
-        sys.modules.pop("tinycudann", None)
-        sys.modules.pop("nerfacc", None)
-    QueryOutput = ref.qio.QueryOutput
+def closed_form_scene(QueryOutput):
+    """The stand-in for the scene representation both sides render: a Gaussian blob whose density depends on the frame."""
 
     class Scene:
         def density(self, q):
@@ -297,116 +224,107 @@ def test_prune_and_render_glue_against_the_reference(ref):
         def __call__(self, q):
             return QueryOutput(density=self.density(q).density, radiance=torch.sigmoid(3.0 * q.positions + q.directions))
 
-    frames = tuple(range(15, 27))
-    b = synthetic_rays(64, 40, frames, ragged=True, seed=8)
+    return Scene()
+
+
+def prune_render_rays():
+    from helpers import synthetic_rays
+
+    return synthetic_rays(64, 40, tuple(range(15, 27)), ragged=True, seed=8)
+
+
+def prune_render_background():
+    return torch.rand(64, 3, generator=torch.Generator().manual_seed(1))
+
+
+def merge_render_parts():
+    g = torch.Generator().manual_seed(9)
+    return [(torch.rand(n, 3, generator=g), torch.rand(n, 1, generator=g)) for n in (3, 0, 5)]
+
+
+def test_prune_and_render_glue_against_the_reference(ref):
+    """The reference's own prune_samples / render / merge_render_outputs (volume_rendering.py:26-150), run on the CPU with
+    `nerfacc` replaced by the oracle's restatement of its three functions and a closed-form stand-in for the scene
+    representation, against the oracle: pins everything the oracle restates AROUND nerfacc (positions, jitter, alpha,
+    t_ends = t + step, mask application, background blend, output shapes).  nerfacc's own arithmetic stays unpinned."""
+    from humanrf_b200.scene_representation.query_io import QueryOutput
+    from humanrf_b200.volume_rendering import RenderOutput as OurRenderOutput
+    from oracle import rendering as R
+
+    doc, arrays = ref
+    b = prune_render_rays()
     o, d, fr, ri = b["o"], b["d"], b["frames"].view(-1, 1), b["ri"]
-
-    def batch(t):
-        return ref.ib.InputBatch(ray_origins=o, ray_directions=d, frame_numbers=fr, unique_frame_numbers=torch.unique(fr).view(-1, 1),
-                                 camera_numbers=torch.zeros_like(fr), sample_distances=t.clone().view(-1, 1), ray_indices=ri.clone(),
-                                 rgba=b["rgba"], width=8, height=8)
-
-    scene = Scene()
+    scene = closed_form_scene(QueryOutput)
+    bg = prune_render_background()
     for is_training in (False, True):
-        ib = batch(b["t"])
-        torch.manual_seed(5)
-        vr.prune_samples(ib, scene, is_training=is_training)
+        tag = "train" if is_training else "eval"
+        want = {k: torch.from_numpy(arrays[f"render_{tag}_{k}"]) for k in ("t", "ri", "color", "wsum", "color_nobg")}
         torch.manual_seed(5)
         t = b["t"].view(-1, 1) + (torch.rand_like(b["t"].view(-1, 1)) * R.STEP if is_training else 0)
         pos = o[ri] + t * d[ri]
         sigma = scene.density(types.SimpleNamespace(positions=pos, frame_numbers=fr[ri])).density
         keep = R.prune_mask(sigma, ri)
         assert 0 < int(keep.sum()) < keep.numel()
-        assert torch.equal(ib.sample_distances, t[keep]) and torch.equal(ib.ray_indices, ri[keep])
-        assert ib.sample_distances.shape == (int(keep.sum()), 1)
+        assert torch.equal(want["t"], t[keep]) and torch.equal(want["ri"], ri[keep])
+        assert want["t"].shape == (int(keep.sum()), 1)
         # render the survivors
-        bg = torch.rand(64, 3, generator=torch.Generator().manual_seed(1))
-        out = vr.render(ib, scene, bg, is_training=is_training)
         tk, rk = t[keep], ri[keep]
         pk = o[rk] + tk * d[rk]
         q = types.SimpleNamespace(positions=pk, directions=d[rk], frame_numbers=fr[rk])
         col, ws = R.render(tk, scene.density(q).density, scene(q).radiance, rk, 64, bg)
-        assert torch.equal(out.color, col) and torch.equal(out.weights_sum, ws)
-        assert out.color.shape == (64, 3) and out.weights_sum.shape == (64, 1)
-        nobg = vr.render(ib, scene, None, is_training=is_training)
-        assert torch.equal(nobg.color, R.render(tk, scene.density(q).density, scene(q).radiance, rk, 64, None)[0])
+        assert torch.equal(want["color"], col) and torch.equal(want["wsum"], ws)
+        assert want["color"].shape == (64, 3) and want["wsum"].shape == (64, 1)
+        assert torch.equal(want["color_nobg"], R.render(tk, scene.density(q).density, scene(q).radiance, rk, 64, None)[0])
     # merge_render_outputs: same concatenation, same error for a field that is not a tensor
-    parts = [vr.RenderOutput(color=torch.rand(n, 3), weights_sum=torch.rand(n, 1)) for n in (3, 0, 5)]
-    a = vr.RenderOutput.merge_render_outputs(parts)
-    c = OurRenderOutput.merge_render_outputs([OurRenderOutput(color=p.color, weights_sum=p.weights_sum) for p in parts])
-    assert torch.equal(a.color, c.color) and torch.equal(a.weights_sum, c.weights_sum)
-    for cls in (vr.RenderOutput, OurRenderOutput):
-        with pytest.raises(RuntimeError, match="Unknown data type"):
-            cls.merge_render_outputs([cls(color=torch.rand(2, 3))])
+    c = OurRenderOutput.merge_render_outputs([OurRenderOutput(color=a, weights_sum=w) for a, w in merge_render_parts()])
+    assert torch.equal(c.color, torch.from_numpy(arrays["merge_color"]))
+    assert torch.equal(c.weights_sum, torch.from_numpy(arrays["merge_wsum"]))
+    with pytest.raises(RuntimeError) as err:
+        OurRenderOutput.merge_render_outputs([OurRenderOutput(color=torch.rand(2, 3))])
+    assert str(err.value) == doc["merge_render_outputs_error"]
+
+
+SCENE_SIZES, SCENE_EMB = (6, 12, 6), 2
+SCENE_ROWS = 256            # samples whose reference outputs are stored (a fixed subset of the batch)
+
+
+def scene_glue_inputs():
+    """Oracle model and ray batch of the scene-representation glue comparison: (model, positions, directions, frames,
+    cameras, ray batch)."""
+    from helpers import positions_of, synthetic_rays
+    from oracle import field as OF
+
+    frames = tuple(range(15, 15 + sum(SCENE_SIZES)))
+    om = OF.make_model(SCENE_SIZES, frames, seed=5, table_init="trained", bf16=False, table_std=0.5, camera_embedding_dim=SCENE_EMB)
+    b = synthetic_rays(96, 24, frames, ragged=True, seed=12, n_distinct_frames=len(frames))
+    ri = b["ri"]
+    return om, positions_of(b), b["d"][ri], b["frames"][ri].view(-1, 1), b["cams"][ri].view(-1, 1), b
 
 
 def test_scene_representation_glue_against_the_reference(ref):
     """The reference's HumanRF.density / forward and Decomposition4D.forward (humanrf.py:158-208, decomposition4d.py:124-135)
-    executed live, with every tcnn module and the composition extension answering through the ORACLE's restatement of
-    that one module.  What is compared is therefore the glue the oracle restates around them: frame -> segment routing,
-    the +0.5 shift, local time, grid axis selection (xyz, xyt, yzt, xzt), composition call, truncated_exp * density_scale,
-    geometry-feature slicing, (d+1)/2, camera embeddings while training / zeros otherwise.  The reference stores the
-    composed features in fp16, hence the tolerances."""
-    from helpers import positions_of, synthetic_rays
-    from oracle import field as OF
-    from oracle import hashgrid
-
-    sizes, E = (6, 12, 6), 2
-    frames = tuple(range(15, 15 + sum(sizes)))
-    om = OF.make_model(sizes, frames, seed=5, table_init="trained", bf16=False, table_std=0.5, camera_embedding_dim=E)
-    try:
-        ref_model, _ = _import_reference_model()
-        from humanrf_b200.synthetic import MODEL_KW
-
-        theirs = ref_model.HumanRF(sorted_frame_numbers=frames, segment_sizes=sizes, **{**MODEL_KW, "camera_embedding_dim": E})
-    finally:
-        sys.modules.pop("tinycudann", None)
-    import humanrf.scene_representation.decomposition4d as d4
-
-    d4.Decomposition4D.to = lambda self, *a, **k: self                       # the reference parks idle segments on the CPU
-    d4.tensor_composition_native.compose_tensors_forward = \
-        lambda xyz, xyt, yzt, xzt, vectors, coords: OF.compose(xyz.float(), xyt.float(), yzt.float(), xzt.float(), vectors, coords).half()
-    for s, fg in enumerate(theirs.feature_grids):
-        with torch.no_grad():
-            fg.vectors.copy_(om.segments[s].vectors)
-        for k, name in enumerate(("xyz_encoding", "xyt_encoding", "yzt_encoding", "xzt_encoding")):
-            enc = getattr(fg, name)
-            enc.forward = (lambda x, s=s, k=k: hashgrid.encode(om.segments[s].grids[k], x.float(), om.segments[s].log2T).half())
-    theirs.sigma_net.forward = lambda f: torch.relu(f.float() @ om.w_sigma[0].t()) @ om.w_sigma[1].t()
-
-    def color_net(x):                                                        # [ (d+1)/2 | geo 15 | embedding E ] -> rgb
-        d, rest = x[:, :3].float() * 2 - 1, x[:, 3:].float()
-        inp = torch.cat((OF.sh4(d), rest, torch.ones((x.shape[0], 48 - 16 - rest.shape[1]))), dim=1)
-        w1, w2, w3 = om.w_color
-        h = torch.relu(torch.relu(inp @ w1.t()) @ w2.t())
-        return torch.sigmoid((h @ w3.t())[:, :3])
-
-    theirs.color_net.forward = color_net
-    with torch.no_grad():
-        theirs.camera_embeddings.weight.copy_(om.camera_embeddings)
-
-    b = synthetic_rays(96, 24, frames, ragged=True, seed=12, n_distinct_frames=len(frames))
-    pos, ri = positions_of(b), b["ri"]
-    dirs, fr, cams = b["d"][ri], b["frames"][ri].view(-1, 1), b["cams"][ri].view(-1, 1)
+    as run with every tcnn module and the composition extension answering through the ORACLE's restatement of that one
+    module, against the oracle.  What is compared is therefore the glue the oracle restates around them: frame -> segment
+    routing, the +0.5 shift, local time, grid axis selection (xyz, xyt, yzt, xzt), composition call,
+    truncated_exp * density_scale, geometry-feature slicing, (d+1)/2, camera embeddings while training / zeros
+    otherwise.  The reference stores the composed features in fp16, hence the tolerances."""
+    arrays = ref[1]
+    om, pos, dirs, fr, cams, b = scene_glue_inputs()
     touched = set(om.f2s[b["frames"].numpy()].tolist())
     assert len(touched) == 3                                                 # all three segments are exercised
+    rows = torch.from_numpy(arrays["scene_rows"])
+    assert rows.numel() == SCENE_ROWS
+    radiance = {}
     for is_training in (True, False):
-        q = ref.qio.QueryInput(is_training=is_training, positions=pos, directions=dirs, frame_numbers=fr,
-                               unique_frame_numbers=torch.unique(b["frames"]).view(-1, 1), camera_numbers=cams)
+        tag = "train" if is_training else "eval"
         with torch.no_grad():
-            out = theirs(q)
-            dens = theirs.density(q)
             sigma, geo, rgb = om.forward(pos, dirs, fr.view(-1), cams.view(-1) if is_training else None)
-        assert out.density.shape == sigma.shape and out.geometry_features.shape == (pos.shape[0], 15) and out.radiance.shape == rgb.shape
-        assert torch.equal(out.density, dens.density)
-        rel = ((out.density - sigma).abs() / sigma.abs().clamp_min(1e-3)).max().item()
-        dg = (out.geometry_features.float() - geo).abs().max().item()
-        dc = (out.radiance - rgb).abs().max().item()
+        assert ref[0]["scene_shapes"][tag] == [list(sigma.shape), [pos.shape[0], 15], list(rgb.shape)]
+        density, geometry, radiance[tag] = (torch.from_numpy(arrays[f"scene_{tag}_{k}"]) for k in ("density", "geometry", "radiance"))
+        rel = ((density - sigma[rows]).abs() / sigma[rows].abs().clamp_min(1e-3)).max().item()
+        dg = (geometry.float() - geo[rows]).abs().max().item()
+        dc = (radiance[tag] - rgb[rows]).abs().max().item()
         print(f"is_training={is_training}: density rel {rel:.2e}, geometry abs {dg:.2e}, radiance abs {dc:.2e}")
         assert rel < 2e-3 and dg < 2e-3 and dc < 1e-3       # measured 5e-5 / 5e-5 / 5e-6 (the fp16 feature buffer)
     # the embedding really is dropped at evaluation: the two passes differ in radiance only
-    q_eval = ref.qio.QueryInput(is_training=False, positions=pos, directions=dirs, frame_numbers=fr,
-                                unique_frame_numbers=torch.unique(b["frames"]).view(-1, 1), camera_numbers=cams)
-    q_train = dataclasses.replace(q_eval, is_training=True)
-    with torch.no_grad():
-        assert (theirs(q_eval).radiance - theirs(q_train).radiance).abs().max() > 1e-3
+    assert (radiance["eval"] - radiance["train"]).abs().max() > 1e-3
