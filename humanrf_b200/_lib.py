@@ -47,7 +47,7 @@ class Samples(C.Structure):
 
 
 class SegmentGrads(C.Structure):
-    _fields_ = [("grid", vp * 4), ("vectors", vp), ("vectors_t", vp)]
+    _fields_ = [("grid", vp * 4), ("vectors", vp)]
 
 
 class AdamTensor(C.Structure):
@@ -107,7 +107,6 @@ _SIGNATURES = {
     "hrf_adam_step": (C.c_int, [vp, vp, vp, vp, vp, i64, f32, f32, f32, f32, C.c_int, f32, vp]),
     "hrf_cast_bf16": (C.c_int, [vp, vp, i64, vp]),
     "hrf_transpose_vectors": (C.c_int, [vp, vp, C.c_int, vp]),
-    "hrf_fold_vector_grads": (C.c_int, [vp, vp, C.c_int, vp]),
     "hrf_occupancy_from_masks": (C.c_int, [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]),
     "hrf_occupancy_union_count": (C.c_int, [vp, vp, i64, vp, vp]),
     "hrf_selftest_umma": (C.c_int, [vp, vp, vp, C.c_int, C.c_int, C.c_int, u32, u32, u32, u32, u32, u32, u32, u32,

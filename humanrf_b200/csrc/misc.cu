@@ -136,7 +136,7 @@ __global__ void __launch_bounds__(128, 1) selftest_umma_kernel(const SelfTestArg
 using namespace hrf;
 
 extern "C" const char* hrf_last_error(void) { return g_last_error.c_str(); }
-extern "C" int hrf_version(void) { return 1; }
+extern "C" int hrf_version(void) { return 2; }
 extern "C" int hrf_device_info(int* out3) {
   int dev = 0;
   HRF_CUDA(cudaGetDevice(&dev));

@@ -20,21 +20,6 @@ __global__ void transpose_vectors_kernel(const float* __restrict__ v, float* __r
   if (i < (int64_t)4 * vr * 32) vt[vectors_t_index(i, vr)] = v[i];
 }
 
-// gradient accumulated by the scatter in the transposed layout -> added to the [4, VR, 32] gradient, scratch re-zeroed
-__global__ void fold_vector_grads_kernel(float* __restrict__ gt, float* __restrict__ g, int vr) {
-  const int64_t i = 2 * ((int64_t)blockIdx.x * blockDim.x + threadIdx.x);      // a feature pair = one level of one row
-  if (i >= (int64_t)4 * vr * 32) return;
-  float2* src = reinterpret_cast<float2*>(gt + vectors_t_index(i, vr));
-  const float2 v = *src;
-  if (v.x != 0.f || v.y != 0.f) {
-    float2* dst = reinterpret_cast<float2*>(g + i);
-    float2 o = *dst;
-    o.x += v.x, o.y += v.y;
-    *dst = o;
-    *src = make_float2(0.f, 0.f);
-  }
-}
-
 __device__ __forceinline__ float block_sum_256(float v) {
   __shared__ float part[8];
 #pragma unroll
@@ -165,15 +150,6 @@ extern "C" int hrf_transpose_vectors(const float* vectors, float* vectors_t, int
   HRF_REQUIRE(vectors != nullptr && vectors_t != nullptr && vec_res >= 1, "bad argument");
   const int64_t n = (int64_t)4 * vec_res * 32;
   transpose_vectors_kernel<<<(unsigned)((n + 255) / 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(vectors, vectors_t, vec_res);
-  HRF_CHECK_LAUNCH();
-  return 0;
-}
-
-extern "C" int hrf_fold_vector_grads(float* vectors_t_grad, float* vectors_grad, int vec_res, void* stream) {
-  HRF_REQUIRE(vectors_t_grad != nullptr && vectors_grad != nullptr && vec_res >= 1, "bad argument");
-  HRF_REQUIRE(((reinterpret_cast<uintptr_t>(vectors_t_grad) | reinterpret_cast<uintptr_t>(vectors_grad)) & 7u) == 0, "8-byte alignment");
-  const int64_t pairs = (int64_t)4 * vec_res * 16;
-  fold_vector_grads_kernel<<<(unsigned)((pairs + 255) / 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(vectors_t_grad, vectors_grad, vec_res);
   HRF_CHECK_LAUNCH();
   return 0;
 }

@@ -27,7 +27,6 @@ running the reference's trainer.py unchanged.
 from __future__ import annotations
 
 import ctypes as C
-import os
 from typing import List, Optional
 
 import numpy as np
@@ -100,17 +99,6 @@ class FusedTrainer:
             for k in range(4):
                 sg[s_].grid[k] = self.grad_views[5 * s_ + k].data_ptr()
             sg[s_].vectors = self.grad_views[5 * s_ + 4].data_ptr()
-        # HRF_VECGRAD_T=1 (experiment, off): the scatter accumulates the vector-row gradients in a transposed scratch
-        # ([4][16][VR][2]: the rows neighbouring samples touch share 128-byte lines) and hrf_fold_vector_grads adds it into
-        # the bucket before Adam / the exchange read the gradient.  Measured on B200 (profiles/r2n_*): L2 RED requests
-        # 141 M -> 118 M, L1TEX 73 -> 57 %, L2 62 -> 50 % -- and the kernel SLOWER, 1.02 -> 1.09 ms: packing the adds of
-        # neighbouring lanes into the same lines makes them queue behind each other in the L2's atomic units.
-        self.vec_grad_t = None
-        if os.environ.get("HRF_VECGRAD_T", "0") == "1":
-            vn = self.grad_views[4].numel()
-            self.vec_grad_t = torch.zeros(S * vn, dtype=torch.float32, device=dev)
-            for s_ in range(S):
-                sg[s_].vectors_t = self.vec_grad_t[s_ * vn:(s_ + 1) * vn].data_ptr()
         self.sg_dev = _device_struct_array([sg], dev)
         i = 5 * S
         self.mlp_grad = self.grad[self.slices[i][0]:self.slices[i + 1][1]]   # sigma params then colour params, contiguous
@@ -376,7 +364,7 @@ class FusedTrainer:
         else:
             L.check(lib.hrf_field_backward_tables(C.byref(nat.field), C.byref(samples), self.sg_dev.data_ptr(), egrid, L.ptr(src),
                                                   egrid_stride, ws.data_ptr(), 0, 4, L.stream()))
-            launches += 8 + self._fold_vector_grads()
+            launches += 8
             if bwd_events is not None:
                 bwd_events[1].record()
             mark("scatter")
@@ -386,16 +374,6 @@ class FusedTrainer:
         if return_loss:
             return float(loss.item())
         return launches
-
-    def _fold_vector_grads(self) -> int:
-        if self.vec_grad_t is None:
-            return 0
-        lib, S = L.lib(), self.model.num_segments
-        vn = self.grad_views[4].numel()
-        for s_ in range(S):
-            L.check(lib.hrf_fold_vector_grads(self.vec_grad_t[s_ * vn:(s_ + 1) * vn].data_ptr(), self.grad_views[5 * s_ + 4].data_ptr(),
-                                              self.model.feature_grids[0].vectors.shape[1], L.stream()))
-        return S
 
     def _exchange_and_adam(self) -> int:
         lib = L.lib()
@@ -434,8 +412,6 @@ class FusedTrainer:
         for k in range(4):
             L.check(lib.hrf_field_backward_tables(C.byref(nat.field), C.byref(samples), self.sg_dev.data_ptr(), egrid, L.ptr(src),
                                                   egrid_stride, ws.data_ptr(), k, 1, L.stream()))
-            if k == 3:
-                self._fold_vector_grads()     # (the vector gradients are complete after the last grid's launch)
             ev = torch.cuda.Event()
             ev.record(main)
             with torch.cuda.stream(side):

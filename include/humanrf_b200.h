@@ -230,14 +230,6 @@ int hrf_composite_backward(const float* sigma, const float* rgb, const float* sa
 typedef struct {
   float* grid[4];                    /* [n_entries,2] fp32, same order as hrf_segment.grid */
   float* vectors;                    /* [4, vec_res, 32] fp32 */
-  /* Optional scratch in the transposed layout of hrf_segment.vectors_t, [4 axes][16 levels][vec_res][2], zeroed by the
-   * caller once.  When non-NULL the default scatter generation accumulates the vector-row gradient THERE instead of in
-   * `vectors`: the two tap rows of a sample, and the rows of the neighbouring samples of a ray, then share 128-byte lines
-   * (16 rows of one level per line instead of one row of 16 levels): 16 % fewer L2 RED requests per launch, but measured
-   * 6 % SLOWER on B200 (same-line adds queue in the L2 atomic units), so humanrf_b200.training leaves it NULL by default.
-   * The caller folds it back with hrf_fold_vector_grads before anything reads `vectors`.  The other scatter
-   * generations ignore the field and add into `vectors` directly, so the fold is always correct. */
-  float* vectors_t;
 } hrf_segment_grads;
 
 int hrf_field_backward(const hrf_field* f, const hrf_samples* s, const hrf_segment_grads* seg_grads /* device array */,
@@ -295,9 +287,6 @@ int hrf_adam_step(float* param, float* exp_avg, float* exp_avg_sq, const float* 
 int hrf_cast_bf16(const float* src, void* dst_bf16, int64_t n, void* stream);
 /* vectors [4, vec_res, 32] -> vectors_t [4, 16, vec_res, 2] (hrf_segment.vectors_t) */
 int hrf_transpose_vectors(const float* vectors, float* vectors_t, int vec_res, void* stream);
-/* vectors_grad[i] += vectors_t_grad[transposed index of i]; vectors_t_grad is left zeroed (ready for the next step).
- * Both [4 * vec_res * 32] fp32. */
-int hrf_fold_vector_grads(float* vectors_t_grad, float* vectors_grad, int vec_res, void* stream);
 
 /* All parameter tensors of a model in ONE launch (the per-tensor entry point above costs one launch per tensor: 23
  * for a single segment).  tensors: device array of descriptors; a tensor whose *active flag is 0 is skipped entirely

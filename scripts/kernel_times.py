@@ -86,11 +86,6 @@ def main():
             sg[s_].grid[k] = grads[5 * s_ + k].data_ptr()
         sg[s_].vectors = grads[5 * s_ + 4].data_ptr()
     sg_dev = torch.from_numpy(np.frombuffer(bytes(sg), dtype=np.uint8).copy()).to(dev)
-    # the same with the vector-row gradient accumulated in the transposed scratch (FusedTrainer's default) + the fold
-    vts = [torch.zeros_like(grads[5 * s_ + 4]).reshape(-1) for s_ in range(model.num_segments)]
-    for s_ in range(model.num_segments):
-        sg[s_].vectors_t = vts[s_].data_ptr()
-    sg_t_dev = torch.from_numpy(np.frombuffer(bytes(sg), dtype=np.uint8).copy()).to(dev)
     d_mlp = torch.zeros(model.mlp_grad_elems, device=dev)
     ws = torch.empty(n * 40, device=dev)
     egrid = feat.data_ptr() + 64 * n
@@ -112,13 +107,6 @@ def main():
 
     timeit("MLP-only forward from features (survivors)", lambda: nat.forward_from_features(s, feat, None))
     timeit("table scatter, saved egrid", lambda: scatter(egrid))
-
-    def scatter_t():
-        L.check(lib.hrf_field_backward_tables(C.byref(nat.field), C.byref(s), sg_t_dev.data_ptr(), egrid, None, 0, ws.data_ptr(), 0, 4, L.stream()))
-        for s_ in range(model.num_segments):
-            L.check(lib.hrf_fold_vector_grads(vts[s_].data_ptr(), grads[5 * s_ + 4].data_ptr(), grads[5 * s_ + 4].shape[1], L.stream()))
-
-    timeit("table scatter, saved egrid, transposed vector grads + fold", scatter_t)
     timeit("table scatter, re-gather tables", lambda: scatter(None))
     timeit("table scatter, saved egrid (L2 warm)", lambda: scatter(egrid), cold=False)
     timeit("backward MLP kernel (L2 warm)", bwd_mlp, cold=False)
