@@ -11,5 +11,6 @@ error behaviour) on top of the C ABI in include/humanrf_b200.h:
   actorshq/dataset/native/occupancy_grid.cu (pybind)   -> humanrf_b200.dataset.occupancy_grid_native
   humanrf/scene_representation/native/tensor_composition.cu -> humanrf_b200.scene_representation.tensor_composition_native
   humanrf/utils/{activation,loss}.py                   -> humanrf_b200.utils
+  actorshq/evaluation/evaluate.py (PSNR, SSIM)         -> humanrf_b200.evaluation.evaluate
 """
 __version__ = "0.1.0"

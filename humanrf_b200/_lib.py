@@ -109,6 +109,9 @@ _SIGNATURES = {
     "hrf_transpose_vectors": (C.c_int, [vp, vp, C.c_int, vp]),
     "hrf_occupancy_from_masks": (C.c_int, [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]),
     "hrf_occupancy_union_count": (C.c_int, [vp, vp, i64, vp, vp]),
+    "hrf_mask_bbox": (C.c_int, [vp, C.c_int, C.c_int, vp, vp]),
+    "hrf_image_metrics_workspace_bytes": (i64, [C.c_int, C.c_int]),
+    "hrf_image_metrics": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, i64, vp, f32, vp, C.c_int, vp, vp, vp]),
     "hrf_selftest_umma": (C.c_int, [vp, vp, vp, C.c_int, C.c_int, C.c_int, u32, u32, u32, u32, u32, u32, u32, u32,
                                     C.c_int, vp]),
 }

@@ -370,6 +370,25 @@ int hrf_occupancy_union_count(void* cluster_bits /* ceil(n/32) u32, caller-zeroe
                               int64_t num_voxels, int64_t* count_dev, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Validation metrics (humanrf/trainer.py:373-419 and actorshq/evaluation/evaluate.py:76-85 without LPIPS), all on the
+ * device with no host read.
+ * hrf_mask_bbox: box = cv2.boundingRect(mask > 0) as int32 (x, y, w, h); an empty mask gives (0, 0, 0, 0).
+ * hrf_image_metrics: im1 / im2 are [height, width, 3] images (fp32, or uint8 when is_uint8), rows row_stride elements
+ * apart, read as value / data_range.  what bit 0: SSIM over the ROI (roi = device (x, y, w, h) clipped to the image,
+ * NULL = whole image) with skimage's defaults as the reference calls structural_similarity: 7x7 uniform window,
+ * sample covariance, K1 = 0.01, K2 = 0.03, map cropped by 3 pixels, mean of the channel means; a ROI narrower or
+ * shorter than 7 gives NaN.  what bit 1: PSNR over the whole image, -10 log10 of the per-pixel channel-mean squared
+ * error averaged over the pixels with psnr_mask != 0 (psnr_mask [height, width] or NULL = all; needs
+ * row_stride == 3 * width).  out[4] (device): SSIM, PSNR, summed squared error, pixel count; what is not computed is
+ * NaN.  workspace: hrf_image_metrics_workspace_bytes(height, width) bytes; results are bitwise reproducible.
+ * ---------------------------------------------------------------------------------------- */
+int hrf_mask_bbox(const uint8_t* mask /* [height, width] */, int height, int width, int32_t* box /* [4] */, void* stream);
+int64_t hrf_image_metrics_workspace_bytes(int height, int width);
+int hrf_image_metrics(const void* im1, const void* im2, int is_uint8, int height, int width, int64_t row_stride,
+                      const int32_t* roi, float data_range, const uint8_t* psnr_mask, int what, double* out,
+                      void* workspace, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Self tests (used by tests/ only): one 128xN x K tcgen05 MMA with caller-chosen descriptor
  * fields, to pin the shared-memory descriptor encoding on real hardware.
  * ---------------------------------------------------------------------------------------- */
